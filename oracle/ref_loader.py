@@ -211,3 +211,75 @@ class ReferenceCodebookNHWC:
     def decode_code(self, codes, training=False):
         with torch.no_grad():
             return self.model.decode_code(torch.as_tensor(codes).as_subclass(torch.Tensor).long()).permute(0, 2, 3, 1).contiguous()
+
+
+def load_reference_generate_codes():
+    """commands/generate_codes.py loaded as shipped, with stand-ins for what is not on this path: `webdataset.filters` (three generators
+    restating the documented behaviour of map_ / unbatched_ / batched_ with the default collation), aparse.click, viewformer.data
+    .transform_dataset; TensorFlow is made un-importable for the duration so that the script's own `except ImportError` branch runs."""
+    import numpy as np
+    load_reference_modules()
+    ap = sys.modules["aparse"]
+    if not hasattr(ap, "click"):                          # the same stand-ins load_reference_evaluate installs
+        ap.click = types.SimpleNamespace(command=lambda *a, **k: (lambda f: f))
+    if not hasattr(ap, "ConditionalType"):
+        ap.ConditionalType = lambda name, table, default=None: typing.Any
+    utils = sys.modules["viewformer.utils"]
+    if not hasattr(utils, "SplitIndices"):
+        utils.SplitIndices = object
+    data = sys.modules.get("viewformer.data")
+    if data is None:
+        data = types.ModuleType("viewformer.data")
+        data.__path__ = []
+        sys.modules["viewformer.data"] = data
+    data.transform_dataset = lambda *a, **k: None
+
+    def collate(samples):
+        cols = list(zip(*samples))
+        out = []
+        for c in cols:
+            if isinstance(c[0], (int, float)):
+                out.append(np.array(list(c)))
+            elif isinstance(c[0], torch.Tensor):
+                out.append(torch.stack(list(c)))
+            elif isinstance(c[0], np.ndarray):
+                out.append(np.array(list(c)))
+            else:
+                out.append(list(c))
+        return out
+
+    def map_(data, f):
+        for s in data:
+            yield f(s)
+
+    def unbatched_(data):
+        for s in data:
+            for i in range(len(s[0])):
+                yield tuple(x[i] for x in s)
+
+    def batched_(data, batchsize=20, partial=True):
+        batch = []
+        for s in data:
+            if len(batch) >= batchsize:
+                yield collate(batch)
+                batch = []
+            batch.append(s)
+        if batch and (len(batch) == batchsize or partial):
+            yield collate(batch)
+
+    wds = types.ModuleType("webdataset")
+    wds.filters = types.SimpleNamespace(map_=map_, unbatched_=unbatched_, batched_=batched_)
+    saved_wds, saved_tf = sys.modules.get("webdataset"), sys.modules.pop("tensorflow", None)
+    sys.modules["webdataset"] = wds
+    sys.modules["tensorflow"] = None                      # `import tensorflow` -> ImportError, as on a torch-only machine
+    try:
+        path = os.path.join(REFERENCE_ROOT, "viewformer", "commands", "generate_codes.py")
+        spec = importlib.util.spec_from_file_location("viewformer_commands_generate_codes_ref", path)
+        m = importlib.util.module_from_spec(spec)
+        spec.loader.exec_module(m)
+    finally:
+        if saved_tf is not None:
+            sys.modules["tensorflow"] = saved_tf
+        else:
+            sys.modules.pop("tensorflow", None)
+    return m, (lambda: sys.modules.__setitem__("webdataset", saved_wds) if saved_wds is not None else sys.modules.pop("webdataset", None))

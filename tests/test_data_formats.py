@@ -119,102 +119,19 @@ def test_frames_feature_png_roundtrip(tmp_path):
     assert np.array_equal(np.asarray(ex["cameras"], np.float32).reshape(3, 7), cams)
 
 
-def _load_reference_generate_codes():
-    """commands/generate_codes.py loaded as shipped, with stand-ins for what is not on this path: `webdataset.filters` (three generators
-    restating the documented behaviour of map_ / unbatched_ / batched_ with the default collation), aparse.click, viewformer.data
-    .transform_dataset; TensorFlow is made un-importable for the duration so that the script's own `except ImportError` branch runs."""
-    import importlib.util
-    import sys
-    import types
-    from oracle import ref_loader
-    ref_loader.load_reference_modules()
-    import typing
-    ap = sys.modules["aparse"]
-    if not hasattr(ap, "click"):                          # the same stand-ins oracle/ref_loader.py::load_reference_evaluate installs
-        ap.click = types.SimpleNamespace(command=lambda *a, **k: (lambda f: f))
-    if not hasattr(ap, "ConditionalType"):
-        ap.ConditionalType = lambda name, table, default=None: typing.Any
-    utils = sys.modules["viewformer.utils"]
-    if not hasattr(utils, "SplitIndices"):
-        utils.SplitIndices = object
-    data = sys.modules.get("viewformer.data")
-    if data is None:
-        data = types.ModuleType("viewformer.data")
-        data.__path__ = []
-        sys.modules["viewformer.data"] = data
-    data.transform_dataset = lambda *a, **k: None
-
-    def collate(samples):
-        cols = list(zip(*samples))
-        out = []
-        for c in cols:
-            if isinstance(c[0], (int, float)):
-                out.append(np.array(list(c)))
-            elif isinstance(c[0], torch.Tensor):
-                out.append(torch.stack(list(c)))
-            elif isinstance(c[0], np.ndarray):
-                out.append(np.array(list(c)))
-            else:
-                out.append(list(c))
-        return out
-
-    def map_(data, f):
-        for s in data:
-            yield f(s)
-
-    def unbatched_(data):
-        for s in data:
-            for i in range(len(s[0])):
-                yield tuple(x[i] for x in s)
-
-    def batched_(data, batchsize=20, partial=True):
-        batch = []
-        for s in data:
-            if len(batch) >= batchsize:
-                yield collate(batch)
-                batch = []
-            batch.append(s)
-        if batch and (len(batch) == batchsize or partial):
-            yield collate(batch)
-
-    wds = types.ModuleType("webdataset")
-    wds.filters = types.SimpleNamespace(map_=map_, unbatched_=unbatched_, batched_=batched_)
-    saved_wds, saved_tf = sys.modules.get("webdataset"), sys.modules.pop("tensorflow", None)
-    sys.modules["webdataset"] = wds
-    sys.modules["tensorflow"] = None                      # `import tensorflow` -> ImportError, as on a torch-only machine
-    try:
-        path = os.path.join(ref_loader.REFERENCE_ROOT, "viewformer", "commands", "generate_codes.py")
-        spec = importlib.util.spec_from_file_location("viewformer_commands_generate_codes_ref", path)
-        m = importlib.util.module_from_spec(spec)
-        spec.loader.exec_module(m)
-    finally:
-        if saved_tf is not None:
-            sys.modules["tensorflow"] = saved_tf
-        else:
-            sys.modules.pop("tensorflow", None)
-    return m, (lambda: sys.modules.__setitem__("webdataset", saved_wds) if saved_wds is not None else sys.modules.pop("webdataset", None))
-
-
 def test_latent_code_transformer_equals_the_reference_class():
     """commands/generate_codes.py:20-78 (the reference's LatentCodeTransformer, run as shipped with a stand-in for webdataset's three
-    filters) against data.LatentCodeTransformer on the same scenes with the same stand-in codebook: same scenes out, same codes, same
-    cameras, same encoder batch sizes.  Equal-length scenes: with ragged scenes the reference mis-assigns the carried-over frames (it
-    assumes they belong to a scene as long as the next batch's first one, generate_codes.py:63) — this implementation keeps a queue."""
-    from oracle import ref_loader
-    if not ref_loader.available():
-        pytest.skip("reference sources not present (GPU box)")
-    ref_mod, restore = _load_reference_generate_codes()
+    filters and a stand-in codebook returning the top-left 2x2 pixels of channel 0; stored by oracle/make_golden.py::ref_latent_code_transformer)
+    against data.LatentCodeTransformer on the same scenes with the same stand-in codebook: same scenes out, same codes, same cameras, same
+    encoder batch sizes.  Equal-length scenes: with ragged scenes the reference mis-assigns the carried-over frames (it assumes they belong
+    to a scene as long as the next batch's first one, generate_codes.py:63) — this implementation keeps a queue."""
+    import json
+    from oracle.make_golden import reference_outputs, latent_code_scenes
+    R = reference_outputs()
+    ref = json.loads(str(R["lct.meta"]))
 
     class Cfg:
         image_size, stride, batch_size = 8, 4, 5
-
-    class RefCodebook(torch.nn.Module):
-        config, calls = Cfg, []
-
-        def encode(self, x):                                 # NCHW float in [-1, 1], as _convert_image_type hands it over
-            self.calls.append(len(x))
-            px = ((x[:, 0, :2, :2] + 1) / 2 * 255).round().to(torch.int64)
-            return None, None, px
 
     class OurCodebook:
         config, device, calls = Cfg, "cpu", []
@@ -223,26 +140,18 @@ def test_latent_code_transformer_equals_the_reference_class():
             self.calls.append(len(x))
             return x[:, :2, :2, 0].to(torch.int64)
 
-    scenes = []
-    for i in range(4):
-        fr = np.zeros((6, 8, 8, 3), np.uint8)
-        fr[:, :2, :2, 0] = (10 * i + np.arange(6))[:, None, None]
-        scenes.append(dict(frames=fr, cameras=np.full((6, 7), i, np.float32)))
     import viewformer_b200._lib as L
     orig = L.resize_u8
     L.resize_u8 = lambda x, size, method=None: x            # frames already have the codebook's size; no device in this test
     try:
-        rcb, ocb = RefCodebook(), OurCodebook()
-        ref_tr = ref_mod.LatentCodeTransformer(rcb, batch_size=5, device="cpu")
+        ocb = OurCodebook()
         our_tr = D.LatentCodeTransformer(ocb, batch_size=5)
-        assert ref_tr.update_dataset_info({}) == our_tr.update_dataset_info({}) == {"token_image_size": 2}
+        assert our_tr.update_dataset_info({}) == ref["dataset_info"] == {"token_image_size": 2}
         for feats in (None, ["frames", "cameras"], ["frames", "cameras-gqn"]):
-            assert ref_tr.output_features(feats) == our_tr.output_features(feats)
-        want = list(ref_tr("train", iter([dict(s) for s in scenes])))
-        got = list(our_tr("train", iter([dict(s) for s in scenes])))
+            assert our_tr.output_features(feats) == ref["output_features"][str(feats)]
+        got = list(our_tr("train", iter([dict(s) for s in latent_code_scenes()])))
     finally:
         L.resize_u8 = orig
-        restore()
-    assert len(want) == len(got) == 4 and rcb.calls == ocb.calls == [5, 5, 5, 5, 4]
-    for w, g in zip(want, got):
-        assert np.array_equal(np.asarray(w["codes"]), np.asarray(g["codes"])) and np.array_equal(np.asarray(w["cameras"]), np.asarray(g["cameras"]))
+    assert len(got) == ref["n_scenes"] == 4 and ocb.calls == ref["encoder_calls"] == [5, 5, 5, 5, 4]
+    for i, g in enumerate(got):
+        assert np.array_equal(R[f"lct.codes{i}"], np.asarray(g["codes"])) and np.array_equal(R[f"lct.cameras{i}"], np.asarray(g["cameras"]))

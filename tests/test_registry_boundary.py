@@ -1,7 +1,9 @@
 """The drop-in boundary, exercised through the REAL reference registry (viewformer/models/__init__.py:15-59):
 AutoModelTH.from_config / AutoModel.from_config must hand out viewformer_b200 objects, both with the run-time patch
 (viewformer_b200.compat.install) and with the three shim files of integration/ placed on the package path.
-CPU-only: constructing the model objects touches no device (weights are laid out at load_state_dict)."""
+CPU-only: constructing the model objects touches no device (weights are laid out at load_state_dict).
+The registry tests execute the reference package itself and skip where its sources are absent; the state_dict keys they compare are
+also held to the reference's, stored in tests/golden/reference_outputs.npz, everywhere."""
 import os
 import sys
 
@@ -10,7 +12,7 @@ import pytest
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 from oracle import ref_loader  # noqa: E402
 
-pytestmark = pytest.mark.skipif(not ref_loader.available(), reason="reference sources not present (GPU box)")
+needs_reference = pytest.mark.skipif(not ref_loader.available(), reason="the reference package's sources are not present")
 
 
 def _fresh_registry(extra_paths=()):
@@ -19,6 +21,7 @@ def _fresh_registry(extra_paths=()):
     return ref_loader.load_reference_registry(extra_paths)
 
 
+@needs_reference
 def test_unpatched_registry_returns_reference_class():
     reg = _fresh_registry()
     cfg = reg.load_config({"model": "vqgan", "ch": 32, "ch_mult": [1, 2], "attn_resolutions": [], "image_size": 16, "embed_dim": 8,
@@ -27,6 +30,7 @@ def test_unpatched_registry_returns_reference_class():
     assert type(m).__module__ == "viewformer.models.vqgan_th"
 
 
+@needs_reference
 @pytest.mark.parametrize("how", ["install", "shim_files"])
 def test_registry_hands_out_b200_models(how):
     from viewformer_b200 import compat, VQGAN, MIGT
@@ -53,6 +57,15 @@ def test_registry_hands_out_b200_models(how):
                                                          "num_res_blocks": 1}))
     want = {k for k in ref_model.state_dict() if not k.startswith(("perceptual_loss.", "loss."))}
     assert set(small.expected_keys()) == want
+
+
+def test_b200_codebook_state_dict_keys_are_the_reference_models():
+    """Strict loading both ways needs the b200 codebook to expect exactly the reference VQGAN's state_dict keys (its loss modules aside)."""
+    from oracle.make_golden import REGISTRY_SMALL_VQ, reference_outputs
+    from viewformer_b200 import compat
+    from viewformer_b200.config import VQGANConfig
+    small = compat.VQGAN_TH(VQGANConfig(**REGISTRY_SMALL_VQ))
+    assert sorted(small.expected_keys()) == [str(k) for k in reference_outputs()["vqgan.state_dict_keys"]]
 
 
 def test_tf_flavour_rejects_nchw_input():

@@ -15,14 +15,29 @@ from viewformer_b200.config import VQGANConfig
 
 pytestmark = pytest.mark.gpu
 
+# VF_TRAIN_TC: "1" (default) runs dense layers and 3x3 stride-1 convs on the exact split-fp16 tensor-core GEMM, "0" keeps the whole
+# backward pass on the fp32 CUDA-core kernels (conv_wgrad with Linear layouts, the SIMT tied head and data gradients)
+# Each golden training test below runs on the default path; a *_cuda_core twin runs the same checks, at the same tolerances, with
+# VF_TRAIN_TC=0.
 
-def test_vqgan_training_step_matches_reference(golden_dir):
+
+def test_vqgan_training_step_matches_reference(golden_dir, monkeypatch):
+    _vqgan_training_step_vs_golden(golden_dir, "1", monkeypatch)
+
+
+def test_vqgan_training_step_cuda_core_matches_reference(golden_dir, monkeypatch):
+    _vqgan_training_step_vs_golden(golden_dir, "0", monkeypatch)
+
+
+def _vqgan_training_step_vs_golden(golden_dir, train_tc, monkeypatch):
     from viewformer_b200 import VQGAN
     from viewformer_b200.train import VQGANTrainer
+    monkeypatch.setenv("VF_TRAIN_TC", train_tc)
     g = np.load(os.path.join(golden_dir, "vqgan_train_small.npz"))
     cfg = VQGANConfig(**dict(SMALL_VQ, perceptual_weight=0.0))
     model = VQGAN(cfg, precision="fp32").load_state_dict(synth.make_vqgan_state_dict(cfg, 5))
     tr = VQGANTrainer(model, bucket_bytes=1 << 16)                 # small buckets: exercises the bucket bookkeeping
+    assert tr.use_tc == (train_tc == "1")
     assert len(tr.buckets) > 3
     names = [str(n) for n in g["names"]]
     gen = torch.Generator().manual_seed(99)
@@ -56,7 +71,8 @@ def test_vqgan_training_step_matches_reference(golden_dir):
             err = float((grads[n] - ref).abs().max() / ref.abs().max().clamp_min(1e-4))
             wfull = max(wfull, err)
             assert err < 2e-3, f"step {step} grad {n}: max rel err {err:.3e}"
-        print(f"[train step {step}] gradients: worst norm/projection rel err {worst:.2e} over {len(names)} tensors; worst element-wise {wfull:.2e} over {len(full)} tensors")
+        print(f"[train step {step} VF_TRAIN_TC={train_tc}] gradients: worst norm/projection rel err {worst:.2e} over {len(names)} tensors; "
+              f"worst element-wise {wfull:.2e} over {len(full)} tensors")
         tr.optimizer_step()
         sd = tr.export_state_dict()
         wp = 0.0
@@ -117,12 +133,21 @@ def test_vqgan_training_step_full_size_matches_reference(golden_dir):
     assert abs(float((emb * torch.randn(emb.shape, generator=ge).double()).sum()) - float(g["emb_dot"])) < 2e-4 * float(g["emb_norm"])
 
 
-def test_vqgan_commit_quantizer_training_step_matches_reference(golden_dir):
+def test_vqgan_commit_quantizer_training_step_matches_reference(golden_dir, monkeypatch):
     """``VQGAN(quantizer="commit")`` = the reference's gradient-trained ``Quantize`` (utils_th.py:75-124, beta = 0.25) in place of QuantizeEMA:
     two optimisation steps against tests/golden/vqgan_train_commit_small.npz (the real reference VQGAN with its own Quantize class dropped
     in, oracle/make_golden.py) — loss (1 + beta) * mean((q - z)^2), codes, gradients of every tensor incl. the codebook, post-Adam codebook."""
+    _vqgan_commit_training_step_vs_golden(golden_dir, "1", monkeypatch)
+
+
+def test_vqgan_commit_quantizer_training_step_cuda_core_matches_reference(golden_dir, monkeypatch):
+    _vqgan_commit_training_step_vs_golden(golden_dir, "0", monkeypatch)
+
+
+def _vqgan_commit_training_step_vs_golden(golden_dir, train_tc, monkeypatch):
     from viewformer_b200 import VQGAN
     from viewformer_b200.train import VQGANTrainer
+    monkeypatch.setenv("VF_TRAIN_TC", train_tc)
     g = np.load(os.path.join(golden_dir, "vqgan_train_commit_small.npz"))
     cfg = VQGANConfig(**dict(SMALL_VQ, perceptual_weight=0.0))
     sd = synth.make_vqgan_state_dict(cfg, 5)
@@ -131,6 +156,7 @@ def test_vqgan_commit_quantizer_training_step_matches_reference(golden_dir):
     model = VQGAN(cfg, precision="fp32", quantizer="commit", beta=0.25).load_state_dict(sd)
     assert "quantize.counter" not in model.expected_keys()
     tr = VQGANTrainer(model, bucket_bytes=1 << 16)
+    assert tr.use_tc == (train_tc == "1")
     names = [str(n) for n in g["names"]]
     assert "quantize.embeddings" in names
     gen = torch.Generator().manual_seed(99)
@@ -162,7 +188,7 @@ def test_vqgan_commit_quantizer_training_step_matches_reference(golden_dir):
             ref = torch.from_numpy(g[f"g{step}.{n}"])
             err = float((grads[n] - ref).abs().max() / ref.abs().max().clamp_min(1e-4))
             assert err < (2e-3 if step == 0 else 0.15), f"step {step} grad {n}: max rel err {err:.3e}"
-        print(f"[commit-quantizer train step {step}] gradients: worst norm/projection rel err {worst:.2e} over {len(names)} tensors")
+        print(f"[commit-quantizer train step {step} VF_TRAIN_TC={train_tc}] gradients: worst norm/projection rel err {worst:.2e} over {len(names)} tensors")
         tr.optimizer_step()
         emb = model._w["q"]["emb"].cpu()
         ref = torch.from_numpy(g[f"p{step}.quantize.embeddings"])
@@ -175,19 +201,29 @@ def test_vqgan_commit_quantizer_training_step_matches_reference(golden_dir):
     assert torch.equal(m2.encode(xq)[2], model.encode(xq)[2])
 
 
-def test_migt_training_step_matches_oracle_autograd(golden_dir):
+def test_migt_training_step_matches_oracle_autograd(golden_dir, monkeypatch):
     """MIGT.train_step (migt.py:464-505): three optimisation steps against tests/golden/migt_train_small.npz — gradients from torch
     autograd through the oracle's forward, optimizer / schedule restated from models/utils.py (oracle/make_golden.py).  The fixture is
     reproduced by the reference's own MIGT.train_step executed over oracle/tf_shim.py (tests/test_reference_on_shim.py, CPU, container)."""
+    _migt_training_step_vs_golden(golden_dir, "1", monkeypatch)
+
+
+def test_migt_training_step_cuda_core_matches_oracle_autograd(golden_dir, monkeypatch):
+    _migt_training_step_vs_golden(golden_dir, "0", monkeypatch)
+
+
+def _migt_training_step_vs_golden(golden_dir, train_tc, monkeypatch):
     from viewformer_b200 import MIGT
     from viewformer_b200.train_migt import MIGTTrainer
     from viewformer_b200.config import MIGTConfig
     from oracle.make_golden import MIGT_TRAIN, MIGT_TRAIN_WARMUP
     from oracle import migt_oracle as mo
+    monkeypatch.setenv("VF_TRAIN_TC", train_tc)
     g = np.load(os.path.join(golden_dir, "migt_train_small.npz"))
     cfg = MIGTConfig(**MIGT_TRAIN)
     model = MIGT(cfg, precision="fp32").load_state_dict(synth.make_migt_state_dict(cfg, 9))
     tr = MIGTTrainer(model, warmup_steps=MIGT_TRAIN_WARMUP, bucket_bytes=1 << 18)
+    assert tr.use_tc == (train_tc == "1")
     assert len(tr.buckets) > 2
     names = [str(n) for n in g["names"]]
     gen = torch.Generator().manual_seed(77)
@@ -219,7 +255,7 @@ def test_migt_training_step_matches_oracle_autograd(golden_dir):
             err = float((grads[n] - ref).abs().max() / ref.abs().max().clamp_min(1e-4))
             wfull = max(wfull, err)
             assert err < 2e-3, f"step {step} grad {n}: max rel err {err:.3e}"
-        print(f"[migt train step {step}] gradients: worst norm/projection rel err {worst:.2e} over {len(names)} tensors; worst element-wise {wfull:.2e}")
+        print(f"[migt train step {step} VF_TRAIN_TC={train_tc}] gradients: worst norm/projection rel err {worst:.2e} over {len(names)} tensors; worst element-wise {wfull:.2e}")
         tr.optimizer_step()
         sd = tr.state_dict()
         lr = max(float(g[f"lr{step}"]), 1e-12)
@@ -309,3 +345,128 @@ def test_migt_training_step_full_size_matches_oracle_autograd(golden_dir):
         worst = max(worst, e)
         assert e < 3e-3, f"{n}: |g| {gn:.6e} vs {rn:.6e}, <g,probe> {gd:.6e} vs {rd:.6e}"
     print(f"[migt full-size train step] gradients: worst norm/projection rel err {worst:.2e} over {len(names)} tensors")
+
+
+def _vqgan_grads(train_tc, monkeypatch):
+    from viewformer_b200 import VQGAN
+    from viewformer_b200.train import VQGANTrainer
+    monkeypatch.setenv("VF_TRAIN_TC", train_tc)
+    cfg = VQGANConfig(**dict(SMALL_VQ, perceptual_weight=0.0))
+    tr = VQGANTrainer(VQGAN(cfg, precision="fp32").load_state_dict(synth.make_vqgan_state_dict(cfg, 5)))
+    assert tr.use_tc == (train_tc == "1")
+    loss = float(tr.forward_backward(vq_images(3, cfg.image_size, 2000)))
+    return loss, tr.export_gradients()
+
+
+def _migt_grads(train_tc, monkeypatch):
+    from viewformer_b200 import MIGT
+    from viewformer_b200.train_migt import MIGTTrainer
+    from viewformer_b200.config import MIGTConfig
+    from oracle.make_golden import MIGT_TRAIN, MIGT_TRAIN_WARMUP
+    from oracle import migt_oracle as mo
+    monkeypatch.setenv("VF_TRAIN_TC", train_tc)
+    cfg = MIGTConfig(**MIGT_TRAIN)
+    tr = MIGTTrainer(MIGT(cfg, precision="fp32").load_state_dict(synth.make_migt_state_dict(cfg, 9)), warmup_steps=MIGT_TRAIN_WARMUP)
+    assert tr.use_tc == (train_tc == "1")
+    codes = synth.make_codes(2, 4, n_embed=cfg.n_embeddings, seed=50)
+    cams = mo.normalize_cameras(mo.to_relative_cameras(synth.make_cameras(2, 4, seed=60))[0])
+    loss = float(tr.forward_backward(cams, codes))
+    return loss, tr.gradients()
+
+
+PATHS_TOL = 4e-5        # measured on a B200 (1000 W): VQGAN 7.7e-6 (a GroupNorm gamma), MIGT 1.1e-6
+
+
+@pytest.mark.parametrize("model", ["vqgan", "migt"])
+def test_cuda_core_and_tensor_core_backward_agree(model, monkeypatch):
+    """Both backward paths are fp32-faithful, so on the same weights and batch their gradients agree tensor by tensor far more closely
+    than either agrees with the reference's golden norms.  A bias gradient sum(dy) is formed from the same terms as its weight gradient
+    sum(x dy), so its rounding is measured against the larger of the two: a conv bias in front of a GroupNorm with one channel per
+    group has an exactly-zero true gradient, and both paths hold rounding noise there."""
+    run = _vqgan_grads if model == "vqgan" else _migt_grads
+    loss_tc, g_tc = run("1", monkeypatch)
+    loss_cc, g_cc = run("0", monkeypatch)
+    assert set(g_tc) == set(g_cc)
+    print(f"[{model} backward paths] loss tensor-core {loss_tc:.8f} CUDA-core {loss_cc:.8f}")
+    assert abs(loss_tc - loss_cc) < 1e-5 * abs(loss_tc)
+    errs = {}
+    for n in g_tc:
+        scale = float(g_tc[n].abs().max())
+        if n.endswith(".bias") and n[:-5] + ".weight" in g_tc:
+            scale = max(scale, float(g_tc[n[:-5] + ".weight"].abs().max()))
+        errs[n] = float((g_tc[n] - g_cc[n]).abs().max()) / max(scale, 1e-30)
+    top = sorted(errs.items(), key=lambda kv: -kv[1])[:4]
+    print(f"[{model} backward paths] worst per-tensor max error / max|g| over {len(errs)} tensors: " + ", ".join(f"{n} {e:.2e}" for n, e in top))
+    bad = {n: e for n, e in errs.items() if e >= PATHS_TOL}
+    assert not bad, f"gradients of the two backward paths differ: {bad}"
+
+
+# one tensor per dropout site: embeddings, attention probabilities, attention output, MLP output; plus the pose embedding
+FD_TENSORS = ["wpe.embeddings", "h.0.attn.c_attn.weight", "h.1.attn.c_proj.weight", "h.1.mlp.c_proj.weight", "pose_embedding.c_fc.weight"]
+# measured on a B200 (1000 W): control (dropout 0) 4.0e-3, dropout 0.1 3.7e-3, both at pose_embedding.c_fc.weight; with the attention-
+# output mask of the backward pass taken from the MLP-output site the dropout run reaches 2.0e-2 .. 3.5e-2
+FD_TOL = 1e-2
+
+
+def _migt_fd_errors(dropout):
+    """Central differences of the trainer's own loss along a unit direction per tensor, against <g, v>.  The dropout masks depend only
+    on (seed, iterations, site) and forward_backward does not advance iterations, so every evaluation sees the same masks.
+    The direction is half the normalised analytic gradient, half random: along a purely random direction <g, v> ~ |g| / sqrt(numel),
+    and the step h that moves the loss by 1e-3 of itself (well above its fp32 rounding) leaves the linear regime.  An analytic gradient
+    that is wrong anywhere in the tensor still shows, through both halves."""
+    from viewformer_b200 import MIGT
+    from viewformer_b200.train_migt import MIGTTrainer
+    from viewformer_b200.config import MIGTConfig
+    from oracle.make_golden import MIGT_TRAIN, MIGT_TRAIN_WARMUP
+    from oracle import migt_oracle as mo
+    cfg = MIGTConfig(**dict(MIGT_TRAIN, dropout=dropout))
+    tr = MIGTTrainer(MIGT(cfg, precision="fp32").load_state_dict(synth.make_migt_state_dict(cfg, 9)), warmup_steps=MIGT_TRAIN_WARMUP, seed=3)
+    assert tr.use_tc
+    tr.iterations = 5
+    codes = synth.make_codes(2, 4, n_embed=cfg.n_embeddings, seed=50)
+    cams = mo.normalize_cameras(mo.to_relative_cameras(synth.make_cameras(2, 4, seed=60))[0])
+
+    def loss_at():
+        tr._wsplit = {}                         # as optimizer_step does: the split-fp16 weight copies follow tr.p
+        return float(tr.forward_backward(cams, codes))
+
+    loss0 = loss_at()
+    grads = tr.gradients()
+    gen = torch.Generator().manual_seed(5)
+    errs = {}
+    for name in FD_TENSORS:
+        p = tr.p[name]
+        gd = grads[name].double()
+        r = torch.randn(tuple(p.shape), generator=gen, dtype=torch.float64)
+        v = gd / gd.norm() + r / r.norm()
+        v /= v.norm()
+        gv = float((gd * v).sum())
+        h = 1e-3 * abs(loss0) / abs(gv)
+        orig = p.clone()
+        p.copy_((orig.double() + h * v.to(p.device)).float())
+        lp = loss_at()
+        p.copy_((orig.double() - h * v.to(p.device)).float())
+        lm = loss_at()
+        p.copy_(orig)
+        fd = (lp - lm) / (2 * h)
+        errs[name] = abs(fd - gv) / abs(gv)
+        print(f"[migt FD dropout={dropout}] {name}: <g,v> {gv:.6e} central difference {fd:.6e} (h {h:.2e}) rel err {errs[name]:.2e}")
+    assert loss_at() == loss0                   # the weights are restored
+    return tr, loss0, errs, loss_at
+
+
+def test_migt_dropout_gradients_match_finite_differences():
+    """MIGT with dropout 0.1 (the config default) at all four dropout sites: the analytic gradient of the trainer against central
+    differences of its own loss.  The same harness at dropout 0, where the gradient is validated against the oracle golden, measures
+    the accuracy of the finite differences; the dropout run is held to the same bound.  A missing 1/(1-rate) at one site would move
+    that site's gradients by ~11%, a mask from the wrong site by far more."""
+    _, loss_ctl, errs_ctl, _ = _migt_fd_errors(0.0)
+    tr, loss_do, errs_do, loss_at = _migt_fd_errors(0.1)
+    print(f"[migt FD] worst rel err: control {max(errs_ctl.values()):.2e}, dropout 0.1 {max(errs_do.values()):.2e} (bound {FD_TOL:.0e})")
+    assert max(errs_ctl.values()) < FD_TOL
+    assert max(errs_do.values()) < FD_TOL
+    # the loss is a deterministic function of (weights, batch, seed, iterations): no forward kernel accumulates with atomics
+    assert loss_at() == loss_do
+    assert loss_do != loss_ctl
+    tr.iterations += 1
+    assert loss_at() != loss_do                 # new masks at the next step

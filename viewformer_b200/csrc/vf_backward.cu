@@ -272,7 +272,8 @@ __global__ void adam_kernel(float* __restrict__ p, const float* __restrict__ g, 
 
 // ---- transformer training step (models/migt.py:464-505): LayerNorm / GELU / embedding / loss backward, AdamWeightDecay --------------
 
-// LayerNorm backward, one warp per row (D <= 1024, D % 4 == 0): dx = rstd (dy g - mean(dy g) - xhat mean(dy g xhat)) + add;
+// LayerNorm backward, one warp per row (any D <= 4096: the [2][D] shared partial sums fit the default 48 KB), columns strided over
+// the warp's lanes: dx = rstd (dy g - mean(dy g) - xhat mean(dy g xhat)) + add;
 // dgamma / dbeta partial sums per block in shared memory, then one atomic per column and block
 __global__ void __launch_bounds__(256) layernorm_bwd_kernel(const float* __restrict__ x, const float* __restrict__ dy, const float* __restrict__ gamma,
                                                             const float* __restrict__ add, long long rows, int D, float eps,

@@ -208,15 +208,17 @@ def nhwc_to_nchw(x):
 
 
 def resize_u8(x_u8, size, method=None):
-    """data/_common.py:19-44 (resize_th) for uint8 NHWC images [N,H,W,C] -> [N,size,size,C]: bilinear (align_corners=False) when
-    shrinking, nearest when growing (or the explicit ``method``)."""
+    """data/_common.py:19-62 (resize -> resize_th) for uint8 NHWC images [N,H,W,C] -> [N,size,size,C]: bilinear (align_corners=False)
+    when shrinking, nearest when growing (or the explicit ``method``).  As in the reference, the images come back unchanged when
+    either side already equals ``size`` (resize tests W, resize_th tests H), and the method is chosen by H: a non-square input
+    can stay non-square."""
     lib = load(True)
     _dev(x_u8, torch.uint8)
     n, h, w, c = x_u8.shape
-    if w == size and h == size:
+    if w == size or h == size:
         return x_u8
     if method is None:
-        method = "nearest" if size > w else "bilinear"
+        method = "nearest" if size > h else "bilinear"
     assert method in ("nearest", "bilinear")
     out = torch.empty((n, size, size, c), dtype=torch.uint8, device=x_u8.device)
     _check(lib.vf_resize_u8(_p(x_u8), n, h, w, c, size, size, int(method == "bilinear"), _p(out), _stream()))

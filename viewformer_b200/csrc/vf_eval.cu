@@ -98,8 +98,11 @@ __global__ void __launch_bounds__(256) ssim_u8_kernel(const uint8_t* __restrict_
             }
         // window means of X = x/255 etc. (the reference filters with 1/49 weights in fp32; the integer sums here are exact)
         const float ux = (float)sx / (49.f * 255.f), uy = (float)sy / (49.f * 255.f);
-        const float uxx = (float)sxx / (49.f * 65025.f), uyy = (float)syy / (49.f * 65025.f), uxy = (float)sxy / (49.f * 65025.f);
-        const float vx = cov_norm * (uxx - ux * ux), vy = cov_norm * (uyy - uy * uy), vxy = cov_norm * (uxy - ux * uy);
+        // uxx - ux*ux = (49 sxx - sx^2) / (49^2 255^2): the numerators are formed exactly (|.| < 2^28) and converted once, since
+        // the fp32 difference of the two means cancels on bright, nearly flat windows (an SSIM error of 2e-5 at 250 vs 250|251)
+        const long long nx = 49ll * sxx - (long long)sx * sx, ny = 49ll * syy - (long long)sy * sy, nxy = 49ll * sxy - (long long)sx * sy;
+        const float vscale = 1.f / (2401.f * 65025.f);
+        const float vx = cov_norm * ((float)nx * vscale), vy = cov_norm * ((float)ny * vscale), vxy = cov_norm * ((float)nxy * vscale);
         const float A1 = 2.f * ux * uy + C1, A2 = 2.f * vxy + C2, B1 = ux * ux + uy * uy + C1, B2 = vx + vy + C2;
         acc += (double)((A1 * A2) / (B1 * B2));
     }
@@ -126,8 +129,9 @@ extern "C" int vf_resize_u8(const void* x, int N, int H, int W, int C, int OH, i
 }
 
 extern "C" int vf_image_pair_sums(const void* a, const void* b, int N, int64_t per_image, uint64_t* out, vf_stream_t s) {
-    VF_CHECK_ARG(a && b && out && N >= 0 && per_image > 0, "vf_image_pair_sums: bad args");
-    if (N == 0) return VF_OK;
+    VF_CHECK_ARG(N >= 0 && per_image > 0, "vf_image_pair_sums: bad args");
+    if (N == 0) return VF_OK;                      // empty tensors may carry null pointers
+    VF_CHECK_ARG(a && b && out, "vf_image_pair_sums: null pointer");
     pair_sums_kernel<<<N, 256, 0, vf_s(s)>>>(reinterpret_cast<const uint8_t*>(a), reinterpret_cast<const uint8_t*>(b), per_image,
                                               reinterpret_cast<unsigned long long*>(out));
     VF_CHECK_LAUNCH("vf_image_pair_sums");
@@ -135,10 +139,11 @@ extern "C" int vf_image_pair_sums(const void* a, const void* b, int N, int64_t p
 }
 
 extern "C" int vf_ssim_u8_k(const void* a, const void* b, int N, int H, int W, int C, double K1, double K2, double* out, vf_stream_t s) {
-    VF_CHECK_ARG(a && b && out && N >= 0 && H >= 7 && W >= 7 && C > 0 && N <= 65535, "vf_ssim_u8: bad args (images must be at least 7x7)");
+    VF_CHECK_ARG(N >= 0 && H >= 7 && W >= 7 && C > 0 && N <= 65535, "vf_ssim_u8: bad args (images must be at least 7x7)");
     VF_CHECK_ARG(K1 >= 0.0 && K1 <= 1e3, "vf_ssim_u8: K1 out of range");
     VF_CHECK_ARG(K2 >= 0.0 && K2 <= 1e3, "vf_ssim_u8: K2 out of range");
-    if (N == 0) return VF_OK;
+    if (N == 0) return VF_OK;                      // empty tensors may carry null pointers
+    VF_CHECK_ARG(a && b && out, "vf_ssim_u8: null pointer");
     cudaError_t e = cudaMemsetAsync(out, 0, sizeof(double) * N, vf_s(s));
     if (e != cudaSuccess) { vf_set_error("vf_ssim_u8: memset: %s", cudaGetErrorString(e)); return VF_ERR_CUDA; }
     const long long total = (long long)(H - 6) * (W - 6) * C;

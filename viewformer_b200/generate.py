@@ -103,6 +103,9 @@ def generate_batch_predictions(transformer_model, codebook_model, images, camera
     if images.shape[2] != size or images.shape[3] != size:        # resize_tf (evaluate_transformer.py:104, data/_common.py:19-62)
         img_dev = L.resize_u8(img_dev[:, :n_enc].reshape((-1,) + tuple(img_dev.shape[2:])).contiguous(), size)
         img_dev = img_dev.reshape((B, n_enc) + tuple(img_dev.shape[1:]))
+        if img_dev.shape[2] != size or img_dev.shape[3] != size:      # the rule leaves images with one side == size unchanged
+            raise ValueError(f"{images.shape[2]}x{images.shape[3]} images do not resize to the codebook's {size}x{size} under the dataset "
+                             "resize rule (it returns them unchanged when one side already matches)")
     codes = codebook_model.encode_u8(img_dev, first_views=n_enc).reshape(B, n_enc, side, side)
 
     gen_codes = transformer_model.generate_codes(codes[:, : T - 1], cams_dev)
